@@ -10,13 +10,19 @@ whole attempts, 200x200 RGB-D render, host rewards AND the observation copied to
 hands it to its caller).  Extra objects on the same JSON line (not the headline): `configs` = BASELINE configs 3, 4, 5 as
 specified (SURVEY 8d; config 5 runs in a child process per rank), `qnet` = the a16 forward alone, `learner` = one learn() update.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--legs 3,4,5,qnet,learn]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--legs 3,4,5,qnet,learn] [--dump-outputs DIR]
 Under torchrun every rank owns one GPU and its own envs (weak scaling, no data-path collective).
+--dump-outputs DIR writes what the last timed step left for a caller of the engine (rank 0's environments) as DIR/<name>.npy; the
+inputs are seeded and the engine's result does not depend on timing, so two runs with the same arguments write the same arrays
+and two builds can be compared array by array.
+Nothing is written into the source tree: the fast oracle build goes to a temporary directory.
 """
 import argparse
+import atexit
 import hashlib
 import json
 import os
+import shutil
 import subprocess
 import sys
 import tempfile
@@ -26,12 +32,13 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only, and the benchmark leaves nothing in it
 
 METRIC = "mujoco_substeps_per_sec"
 UNIT = "substeps/s"
 STATE_BYTES_PER_SUBSTEP = 2 * (50 + 44 + 44 + 14) * 8  # fp64 read+write of qpos, qvel, qacc_warmstart, 7 PID inputs, 7 targets (scene A)
 ENGINE_SO = os.path.join(ROOT, "mujoco_rl_ur5_b200", "csrc", "libgrasp_engine.so")
-ORACLE_FAST = os.path.join(ROOT, "oracle", "libgrasp_oracle_fast.so")
+DUMP_MAX_BYTES = 60 * 10**6  # --dump-outputs stays under 64 MB with the .npy headers
 
 
 def measured_peak():
@@ -81,12 +88,18 @@ def lib_sha16(path=ENGINE_SO):
 
 
 def build_fast_oracle():
-    """-O3 -march=native -ffp-contract=fast build of the oracle, compiled on THIS machine (the optimistic CPU baseline)"""
+    """-O3 -march=native -ffp-contract=fast build of the oracle, compiled on THIS machine (the optimistic CPU baseline) in a temporary
+    directory that is removed at exit; returns the library's path, or None if it does not build"""
     try:
-        subprocess.check_call(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "-B", "fast"], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
-        return os.path.exists(ORACLE_FAST)
+        d = tempfile.mkdtemp(prefix="grasp_oracle_fast_")
+        atexit.register(shutil.rmtree, d, True)
+        for f in ("Makefile", "grasp_oracle.c", "orc_math.h"):
+            shutil.copy(os.path.join(ROOT, "oracle", f), d)
+        subprocess.check_call(["make", "-s", "-C", d, "fast"], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+        so = os.path.join(d, "libgrasp_oracle_fast.so")
+        return so if os.path.exists(so) else None
     except Exception:
-        return False
+        return None
 
 
 class ClockSampler:
@@ -181,9 +194,10 @@ def cpu_baseline_single(budget_s=10.0):
     n2, dt2 = _oracle_leg_subprocess(None, half)
     v2 = n2 / dt2
     v3, n3, dt3 = None, 0, 0.0
-    if build_fast_oracle():
+    fast = build_fast_oracle()
+    if fast:
         try:
-            n3, dt3 = _oracle_leg_subprocess(ORACLE_FAST, half)
+            n3, dt3 = _oracle_leg_subprocess(fast, half)
             v3 = n3 / dt3
         except Exception:
             v3 = None
@@ -240,7 +254,7 @@ def run_reference(args):
     cores = hc["usable"]
     fast = build_fast_oracle()
     if fast:
-        os.environ["GRASP_ORACLE_SO"] = ORACLE_FAST  # inherited by the spawned workers
+        os.environ["GRASP_ORACLE_SO"] = fast  # inherited by the spawned workers
     budget = args.ref_step_seconds
     ctx = mp.get_context("spawn")
     with ctx.Pool(cores, initializer=_ref_init) as pool:
@@ -290,6 +304,22 @@ def run_config5_child(args):
            "workspace": "shared memory, CTA per env" if e5.engine.size(9) else "shared memory, warp per env"}
     e5.close()
     print(json.dumps(out), flush=True)
+
+
+def dump_outputs(directory, arrays):
+    """writes each [N, ...] tensor as <directory>/<name>.npy, float32 kept, everything else as float64; above DUMP_MAX_BYTES in all, the
+    same seeded sample of environments (rows) from every array, with their indices in env_index.npy"""
+    arrays = {k: v.detach().cpu().numpy() for k, v in arrays.items()}
+    arrays = {k: v.astype(np.float32 if v.dtype == np.float32 else np.float64) for k, v in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(v.nbytes for v in arrays.values()) // max(n, 1)
+    if n * row_bytes > DUMP_MAX_BYTES:
+        keep = np.sort(np.random.RandomState(0).choice(n, DUMP_MAX_BYTES // (row_bytes + 8), replace=False))
+        arrays = {k: v[keep] for k, v in arrays.items()}
+        arrays["env_index"] = keep.astype(np.float64)
+    os.makedirs(directory, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(directory, k + ".npy"), v)
 
 
 def run_ours(args):
@@ -361,6 +391,12 @@ def run_ours(args):
         kern_evs.append((b, c))
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        qpos, qvel = eng.get_state()
+        result, steps, reward, total = eng.results()
+        dump_outputs(args.dump_outputs, {"qpos": qpos, "qvel": qvel, "targets": eng.get_targets(), "ctrl": eng.get_ctrl(), "result": result,
+                                         "steps": steps, "reward": reward, "total_substeps": total, "grasp_info": eng.grasp_info(),
+                                         "busy": eng.busy(), "status": eng.status()})
     ms = sum(a.elapsed_time(c) for a, c in evs)
     kern_ms = sum(b.elapsed_time(c) for b, c in kern_evs)
     sub1 = env.total_substeps()
@@ -631,6 +667,8 @@ def main():
     ap.add_argument("--scene-b-envs", type=int, default=1024, help="environments per GPU of the config 5 leg")
     ap.add_argument("--scene-b-steps", type=int, default=1, help="timed BatchedGraspEnv.step calls (full grasp attempts) of the config 5 leg")
     ap.add_argument("--ref-step-seconds", type=float, default=3.0, help="--impl reference: wall-time budget per worker and step")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the engine state and results after the last timed step as DIR/<name>.npy (rank 0's environments)")
     ap.add_argument("--oracle-leg", type=float, default=None, help=argparse.SUPPRESS)
     ap.add_argument("--config5-child", type=int, default=None, help=argparse.SUPPRESS)
     ap.add_argument("--config5-offset", type=int, default=0, help=argparse.SUPPRESS)

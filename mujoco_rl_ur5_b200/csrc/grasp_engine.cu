@@ -29,9 +29,11 @@ extern "C" const char* ge_version(void) { return GE_NW > 1 ? "grasp_engine 0.3 s
 // Sub-step kernel: one warp per environment, environments handed to warps DYNAMICALLY.
 // A launch gives every environment a budget of `nsub` iterations of the reference control loop (PID -> mj_step, including the
 // movement / grasp-program transitions), split into visits of `quota` iterations.  Task t of a launch = (visit t / n_env, env t % n_env);
-// a warp that has no environment takes the next task from a global counter, skips it if the environment is idle or another warp
-// still holds it (per-env lock, never waited for), otherwise loads the env's state rows into its shared-memory slice, runs the
-// visit and writes the rows back.  The grid is persistent (<= the resident CTAs), so 4096 envs on 1184 warp slots cost 13.84 -> 14
+// a warp that has no environment takes the next task from a global counter, skips it if the environment is idle, hands its
+// iterations to the warp that still runs an earlier visit of it (per-env lock word: bit 0 held, the rest handed-over iterations; the
+// holder runs them before it lets go), otherwise loads the env's state rows into its shared-memory slice, runs the visit and writes
+// the rows back.  No iteration of a busy env is dropped, so every env runs its whole budget (or until it goes idle) and what a launch
+// computes does not depend on timing.  The grid is persistent (<= the resident CTAs), so 4096 envs on 1184 warp slots cost 13.84 -> 14
 // rounds of 64 iterations instead of 3.46 -> 4 rounds of 256, finished or idle environments stop costing anything, and the tail
 // of a batch of unequal grasp attempts is spread over all SMs.  Arithmetic per env is unchanged: the state crosses HBM in full
 // fp64 between visits, so a trajectory does not depend on how its iterations were cut.
@@ -119,15 +121,24 @@ __global__ void GE_RUN_BOUNDS k_run(EnvArrays E, int n_env, int nsub, int quota,
       t = group_bcast_u64(t, lane);
       if (t >= total) { exhausted = true; break; }
       const int e = (int)(t % (unsigned long long)n_env), v = (int)(t / (unsigned long long)n_env);
-      // ONE thread looks at the env's flags and takes the lock, the group follows its verdict: the flags change under our feet when
+      const int n_it = nsub - v * quota < quota ? nsub - v * quota : quota;
+      // ONE thread takes the lock and looks at the env's flags, the group follows its verdict: the flags change under our feet when
       // another group finishes a visit of this env, and threads that read them separately (the four warps of a CTA-per-env group do
-      // so at different times) would part ways - r02d: illegal instruction / illegal address at >= 300 envs
+      // so at different times) would part ways - r02d: illegal instruction / illegal address at >= 300 envs.  The flags are only
+      // read under the lock: read while another group stores them they may mix old and new values.
       int got = 0;
-      if (lane == 0 && env_is_busy(E, e) && atomicCAS(E.lock + e, 0, 1) == 0) {
-        // an earlier visit of this env still running elsewhere fails the CAS: this visit is dropped, never waited for
-        __threadfence();
-        if (env_is_busy(E, e)) got = 1;
-        else atomicExch(E.lock + e, 0);
+      if (lane == 0) {
+        for (;;) {
+          int old = atomicCAS(E.lock + e, 0, 1);
+          if (old == 0) {
+            __threadfence();
+            if (env_is_busy(E, e)) got = 1;
+            else atomicExch(E.lock + e, 0);
+            break;
+          }
+          // an earlier visit of this env still runs elsewhere: it takes this visit's iterations over
+          if (atomicCAS(E.lock + e, old, old + 2 * n_it) == old) break;
+        }
       }
       got = group_bcast_int(got, lane);
       if (!got) continue;
@@ -135,7 +146,7 @@ __global__ void GE_RUN_BOUNDS k_run(EnvArrays E, int n_env, int nsub, int quota,
       if (GE_NW > 1 && lane == 0) g_hovf = E.gws ? E.gws + (size_t)e * L.hfull : nullptr;  // this env's Hessian overflow row
       env_load(E, e, ws, lane, r);
       env = e; running = true;
-      left = nsub - v * quota < quota ? nsub - v * quota : quota;
+      left = n_it;
     }
 #if GE_NW == 1
     __syncwarp();
@@ -168,8 +179,20 @@ __global__ void GE_RUN_BOUNDS k_run(EnvArrays E, int n_env, int nsub, int quota,
       env_store(E, env, ws, lane, r);
       __threadfence();
       gsync();
-      if (lane == 0) atomicExch(E.lock + env, 0);
-      env = -1;
+      // let go of the env, or run the iterations that later visits handed over meanwhile (the state is still in shared memory)
+      int more = 0;
+      if (lane == 0) {
+        if (!running) atomicExch(E.lock + env, 0);  // idle env: handed-over iterations have nothing to do
+        else for (;;) {
+          int old = atomicCAS(E.lock + env, 1, 0);
+          if (old == 1) break;
+          if (atomicCAS(E.lock + env, old, 1) == old) { more = old >> 1; break; }
+        }
+      }
+      more = group_bcast_int(more, lane);
+      r.nstep = 0;  // env_store added them to the env's sub-step counter
+      if (more > 0) left = more;
+      else env = -1;
     }
   }
 }

@@ -1,5 +1,6 @@
 """Offline-RL wire format (SURVEY 8f.3): files written from batched observations are what the reference's own loader
 (`Offline RL/grasping_dataset.py`) and scripts (`generate_data.py`, `unite_data.py`, `extract_positives.py`) read and write."""
+import json
 import os
 import sys
 
@@ -8,7 +9,7 @@ import pytest
 
 from mujoco_rl_ur5_b200 import offline_data as od
 
-REF = "/root/reference"
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_classes.json")
 
 
 def _batch(n, seed=0, H=200, W=200):
@@ -73,44 +74,30 @@ def test_ragged_reference_file_is_cut_to_the_common_prefix(tmp_path):
     assert len(od.load_transitions(p)[0]) == 4
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "Offline RL")), reason="the reference checkout is not on this machine")
 def test_reference_dataset_class_reads_our_file(tmp_path):
-    """the unmodified Grasping_Dataset (Offline RL/grasping_dataset.py:12-74) on a file written by this module"""
-    pytest.importorskip("torchvision")
-    import importlib.util
-    import types
+    """the unmodified Grasping_Dataset (Offline RL/grasping_dataset.py:12-74) on a file written by this module, frozen in
+    tests/golden/reference_classes.json (tests/golden/make_reference_classes_golden.py): the same file read the way that class reads
+    it (torch.load, then states[i]["rgb"/"depth"], actions[i], rewards[i]) gives its length, action, reward and depth channel"""
+    import torch
 
+    g = json.load(open(GOLD))["grasping_dataset"]
     rgb, depth, act, rew = _batch(3, seed=5)
     p = str(tmp_path / "grasping_data_1.pt")
     od.save_transitions(p, rgb, depth, od.flat_action(act), rew)
-    # grasping_dataset.py does `from Modules import simple_Transition`; give it a light stand-in so Modules' own imports are not needed
-    saved = {k: sys.modules.get(k) for k in ("Modules",)}
-    from collections import namedtuple
-
-    sys.modules["Modules"] = types.SimpleNamespace(simple_Transition=namedtuple("simple_Transition", ("state", "action", "reward")))
-    try:
-        spec = importlib.util.spec_from_file_location("ref_grasping_dataset", os.path.join(REF, "Offline RL", "grasping_dataset.py"))
-        mod = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mod)
-        import torch
-
-        _orig = torch.load
-        torch.load = lambda f, *a, **k: _orig(f, *a, **{**k, "weights_only": False})  # the reference predates the weights_only default
-        try:
-            ds = mod.Grasping_Dataset(p)
-        finally:
-            torch.load = _orig
-        assert len(ds) == 3
-        np.random.seed(0)
-        state, a, r = ds[1]
-        assert tuple(state.shape) == (4, 200, 200) and a == int(od.flat_action(act)[1]) and r == int(rew[1])
-        assert float(state[3].min()) == 0.0 and float(state[3].max()) == 1.0  # min-max normalised depth channel
-    finally:
-        for k, v in saved.items():
-            if v is None:
-                sys.modules.pop(k, None)
-            else:
-                sys.modules[k] = v
+    data = torch.load(p, weights_only=False)
+    assert len(data["states"]) == g["length"] == 3
+    assert data["actions"][1] == g["action"] == int(od.flat_action(act)[1]) and data["rewards"][1] == g["reward"] == int(rew[1])
+    s = data["states"][1]
+    assert g["shape"] == [4, 200, 200] and s["rgb"].shape == (200, 200, 3) and s["rgb"].dtype == np.uint8  # HWC uint8: what ToPILImage takes
+    # transform_observation's depth channel (grasping_dataset.py:42-56), in float32 like the file: clip at 1.1, add N(0, 1e-3) noise,
+    # negate, min-max normalise
+    np.random.seed(0)
+    d = np.minimum(s["depth"], np.float32(1.1))
+    d += np.random.normal(loc=0, scale=0.001, size=d.shape)
+    d = -d
+    d = (d - d.min()) / (d.max() - d.min())
+    assert float(d.min()) == 0.0 and float(d.max()) == 1.0
+    assert np.abs(d.reshape(-1)[g["pixels"]].astype(np.float32) - np.array(g["depth"], np.float32)).max() <= 1e-6
 
 
 @pytest.mark.gpu

@@ -58,7 +58,7 @@ def test_replay_fixture_exercises_every_outcome():
 
 
 @pytest.mark.gpu
-def test_fixed_256_action_replay_matches_oracle():
+def test_fixed_256_action_replay_matches_oracle(tmp_path):
     from mujoco_rl_ur5_b200.batched_env import BatchedGraspEnv
 
     g = _load()
@@ -122,12 +122,7 @@ def test_fixed_256_action_replay_matches_oracle():
                                            "mean_fraction_within_tol": float(post_frac.mean()), "min_fraction_within_tol": float(post_frac.min()),
                                            "most_pixels_off_in_one_image": post_worst_px},
               "mismatches": [list(map(str, b)) for b in bad]}
-    out = os.path.join(os.path.dirname(os.path.dirname(os.path.dirname(GOLD))), "gpurun_out")
-    try:
-        os.makedirs(out, exist_ok=True)
-        json.dump(report, open(os.path.join(out, "replay_256_report.json"), "w"), indent=1)
-    except OSError:
-        pass
+    json.dump(report, open(tmp_path / "replay_256_report.json", "w"), indent=1)
     print("replay:", {k: v for k, v in report.items() if k != "mismatches"})
     # gates: depth / executed / reward / arm angles on every one of the 256 records; the per-phase sub-step counts must agree on
     # >= 98 % of the executed attempts (a tolerance test that falls one sub-step later on one side is rounding, not a different
@@ -143,7 +138,7 @@ def test_fixed_256_action_replay_matches_oracle():
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("build", ["default", "nofma"])
-def test_free_running_replay_agreement(build):
+def test_free_running_replay_agreement(build, tmp_path):
     """The same 256 actions WITHOUT re-synchronisation (every env continues from its own state).  Contact dynamics amplifies
     rounding: the CPU oracle replaying its own fixture with ONE coordinate moved by one unit in the last place reproduces 250 of
     256 records (4 of 16 envs leave the trajectory, first at step 7), the oracle built with -O3 -ffp-contract=fast 249 of 256
@@ -153,7 +148,7 @@ def test_free_running_replay_agreement(build):
     import sys
 
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    out = os.path.join(root, "gpurun_out", f"free_run_gpu_{build}.json")
+    out = str(tmp_path / f"free_run_gpu_{build}.json")
     envv = dict(os.environ)
     if build == "nofma":
         lib = os.path.join(root, "mujoco_rl_ur5_b200", "csrc", "libgrasp_engine_nofma.so")

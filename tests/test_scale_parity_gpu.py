@@ -162,3 +162,46 @@ def test_scene_b_fixture_shape():
     st = np.load(os.path.join(GOLD, "scene_b_attempts.npz"))
     assert len(g["records"]) == 8 and st["qpos0"].shape == (8, 288) and st["qvel0"].shape == (8, 248)
     assert all(r["substeps"] > 1000 for r in g["records"])
+
+
+def _timed_path(n, launches, chunk=256):
+    """bench.py's timed path (idle envs get a seeded random grasp target, then one launch of `chunk` iterations), recording each
+    launch's per-env sub-step increments and whether the env was still busy after it"""
+    import torch
+
+    from mujoco_rl_ur5_b200.batched_env import BatchedGraspEnv
+
+    env = BatchedGraspEnv(n, "A", 0)
+    eng = env.engine
+    env.reset()
+    gen = torch.Generator(device="cuda").manual_seed(30000)
+    steps = []
+    for _ in range(launches):
+        idle = eng.busy() == 0
+        u = torch.rand((n, 3), generator=gen, device="cuda", dtype=torch.float64)
+        coords = torch.stack([-0.2 + 0.4 * u[:, 0], -0.75 + 0.3 * u[:, 1], torch.full((n,), 0.92, device="cuda", dtype=torch.float64)], dim=1)
+        rot = torch.randint(0, 6, (n,), generator=gen, device="cuda", dtype=torch.int32)
+        eng.grasp(coords, rot, 0.91, env_mask=idle.to(torch.uint8))
+        before = eng.results()[3].clone()
+        eng.run_async(chunk)
+        steps.append(((eng.results()[3] - before).cpu().numpy(), eng.busy().cpu().numpy() != 0))
+    qpos, qvel = eng.get_state()
+    out = (qpos.cpu().numpy(), qvel.cpu().numpy(), eng.results()[3].cpu().numpy(), eng.grasp_info().cpu().numpy())
+    env.close()
+    return steps, out
+
+
+@pytest.mark.gpu
+def test_run_async_gives_every_busy_env_its_whole_budget_and_is_reproducible():
+    """k_run hands 32-iteration visits of the envs to whichever warp is free.  An env still busy after a launch must have run all of
+    the launch's iterations (a visit that finds an earlier visit of the same env still running hands its iterations over to it instead
+of being dropped), so that two runs
+    of the same inputs compute the same states bit for bit - at the benchmarked size, where visits of unequal length collide"""
+    n, launches, chunk = 4096, 8, 256
+    steps, first = _timed_path(n, launches, chunk)
+    for inc, busy in steps:
+        assert (inc[busy] == chunk).all(), np.unique(inc[busy], return_counts=True)
+        assert (inc <= chunk).all()
+    _, second = _timed_path(n, launches, chunk)
+    for a, b in zip(first, second):
+        assert np.array_equal(a, b), int((a != b).reshape(n, -1).any(axis=1).sum())
